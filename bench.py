@@ -45,6 +45,7 @@ def emit(line: dict):
 METRIC = "clip+sentence pairs/sec"
 UNIT = "pairs/s"
 CPU_SAMPLE_VIDEOS = 16
+DUMP_LIMIT_BYTES = 64_000_000
 
 
 def parse_args():
@@ -64,7 +65,40 @@ def parse_args():
                     help="e2e host feature storage: fp16_packed = data.PackedFeatureStore (packed valid rows, IEEE fp16, SURVEY 8f-2; "
                          "default); fp32 = the padded fp32 tensors of the reference contract (valid rows staged)")
     ap.add_argument("--no-clocks", action="store_true", help="do not sample clocks (use when running under ncu)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (loss, and the gradient of every net's parameters) as DIR/<name>.npy, "
+                         f"float32, at most {DUMP_LIMIT_BYTES // 10**6} MB in all; the inputs are seeded, so two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload.startswith("cfg5_loss_n")):
+        ap.error("--dump-outputs applies to --impl b200 on the training-step workloads")
+    return args
+
+
+def step_outputs(loss, mgr):
+    """Host copies of what one training step hands its caller: the loss, and per net the gradient of its trainable parameters
+    flattened in named_parameters() order."""
+    import torch as th
+    from coot_videotext_b200.model_retrieval import NET_NAMES
+    out = {"loss": loss.detach().float().reshape(1).cpu().numpy()}
+    for net in NET_NAMES:
+        grads = [p.grad.detach().flatten() for p in mgr.model_dict[net].parameters() if p.requires_grad]
+        out[f"grad_{net}"] = th.cat(grads).float().cpu().numpy()
+    return out
+
+
+def write_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """Writes DIR/<name>.npy.  Above `limit` bytes in all, every array is replaced by the same fixed, seeded sample of its elements
+    (flattened, indices ascending) in proportion to its size, so that runs with the same arguments stay comparable."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > limit:
+            keep = max(1, a.size * limit // total)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def workload_config(wl, n_gpus, input_bytes=None):
@@ -488,6 +522,8 @@ def run_b200(args, wl):
     e1.record()
     sync_all()
     ms = max_over_ranks(e0.elapsed_time(e1))
+    # taken before anything below runs another step (launch count, e2e, profiled pass) and overwrites the gradients
+    outputs = step_outputs(loss, mgr) if (args.dump_outputs and rank == 0) else None
     launches = lib.coot_launch_count() - launches0
     launches_per_step = launches / args.steps
     if launches == 0:  # CUDA-graph replay: the library's launch sites ran once at capture time; count one un-captured step
@@ -575,6 +611,8 @@ def run_b200(args, wl):
                 "dp_graph_mode": getattr(hot, "dp_graph_mode", None) if world > 1 else None,
                 "forward_only": {"value": pairs_local * world * args.steps / (ms_fwd * 1e-3), "unit": UNIT, "ms_per_step": ms_fwd / args.steps},
                 "roofline": roofline, "attention": attention if rank == 0 else None, "cpu_baseline": cpu, "breakdown": breakdown, "loss": float(loss), "pairs_per_step": pairs_local * world}
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         emit(line)
     if world > 1:
         # captured graphs hold NCCL kernels: drop them before leaving, and leave without waiting for communicator destruction

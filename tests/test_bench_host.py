@@ -35,6 +35,25 @@ def test_roofline_blocks_reproduce_committed_line():
         assert attention[n]["ms_per_step"] == pytest.approx(line["breakdown"][n]["ms_per_step"])
 
 
+def test_dumped_outputs_are_whole_under_the_limit_and_a_fixed_sample_above(tmp_path):
+    import numpy as np
+    rng = np.random.default_rng(1)
+    arrays = {"loss": np.float32([1.5]), "grad_a": rng.standard_normal(3000).astype(np.float32),
+              "grad_b": rng.standard_normal((10, 100)).astype(np.float32)}
+    bench.write_outputs(str(tmp_path / "whole"), arrays)
+    for name, a in arrays.items():
+        assert np.array_equal(np.load(tmp_path / "whole" / f"{name}.npy"), a)
+    for run in ("one", "two"):
+        bench.write_outputs(str(tmp_path / run), arrays, limit=8000)
+    total = 0
+    for name, a in arrays.items():
+        s = np.load(tmp_path / "one" / f"{name}.npy")
+        assert s.dtype == np.float32 and np.array_equal(s, np.load(tmp_path / "two" / f"{name}.npy"))
+        assert np.isin(s, a).all()
+        total += s.nbytes
+    assert 0 < total <= 8000
+
+
 def test_cfg5_workload_string():
     pat = r"cfg5_loss_n([\d,]+)(?:_d(\d+))?$"
     assert pat in open(os.path.join(ROOT, "bench.py")).read()

@@ -1,35 +1,29 @@
 """Every reference citation `path.py:line[-line]` in the C header, the oracle and the host layer must point into an existing file of
-the reference tree, inside its length (CPU only; skipped where the reference tree is not available)."""
+the reference tree, inside its length (CPU only).  The file lengths were recorded from the reference tree by
+tests/golden/make_golden_reference_meta.py (tests/golden/reference_line_counts.json)."""
+import json
 import os
 import re
 
-import pytest
-
-from oracle import ref_import
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PAT = re.compile(r"((?:coot|nntrainer|mart|tests_nntrainer|config)/[\w/.]+\.(?:py|yaml)):(\d+)(?:-(\d+))?")
+CITED_DIRS = ("coot", "nntrainer", "mart", "tests_nntrainer", "config")
+PAT = re.compile(r"((?:" + "|".join(CITED_DIRS) + r")/[\w/.]+\.(?:py|yaml)):(\d+)(?:-(\d+))?")
 SOURCES = ["include/coot_sm100.h", "oracle/coot_oracle.py", "oracle/retrieval_oracle.py", "oracle/optim_oracle.py", "oracle/ref_runner.py",
            "DESIGN.md", "INTEGRATION.md", "coot_videotext_b200/model_retrieval.py", "coot_videotext_b200/loss_fn.py",
            "coot_videotext_b200/retrieval.py", "coot_videotext_b200/optimization.py", "coot_videotext_b200/export.py",
            "coot_videotext_b200/data.py", "coot_videotext_b200/h5min.py", "coot_videotext_b200/synthetic.py"]
 
 
-@pytest.mark.skipif(not ref_import.reference_available(), reason="reference tree not available")
 def test_reference_citations_resolve():
-    ref_root = ref_import.REFERENCE_ROOT
-    lengths, bad, total = {}, [], 0
+    lengths = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_line_counts.json")))
+    bad, total = [], 0
     for src in SOURCES:
         text = open(os.path.join(ROOT, src), encoding="utf8").read()
         for m in PAT.finditer(text):
             path, lo, hi = m.group(1), int(m.group(2)), int(m.group(3) or m.group(2))
-            full = os.path.join(ref_root, path)
-            if not os.path.isdir(os.path.join(ref_root, path.split("/")[0])):
-                continue  # the travelling copy oracle/_ref holds coot/, nntrainer/ and config/ only
-            if path not in lengths:
-                lengths[path] = sum(1 for _ in open(full, encoding="utf8", errors="replace")) if os.path.isfile(full) else -1
             total += 1
-            if lengths[path] < 0 or not (1 <= lo <= hi <= lengths[path]):
-                bad.append((src, m.group(0), lengths[path]))
+            n = lengths.get(path, -1)
+            if n < 0 or not (1 <= lo <= hi <= n):
+                bad.append((src, m.group(0), n))
     assert total > 100, total
     assert not bad, bad

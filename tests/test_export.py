@@ -49,8 +49,8 @@ def test_embedding_file_has_the_reference_layout(tmp_path):
 
 
 def test_checkpoint_files_round_trip_with_the_reference_manager(tmp_path):
-    from oracle import ref_import
     from coot_videotext_b200.model_retrieval import RetrievalModelManager
+    from tests.test_nets_cpu import golden_layout, layout, reference_managers
     mine = RetrievalModelManager(vid_feat_dim=64, text_feat_dim=96)
     X.save_checkpoint(tmp_path, 3, mine, opt_state={"optimizer": {"state": {}}, "lr_scheduler": {"step": 5}})
     assert os.path.isfile(tmp_path / "models" / "model_3.pth") and os.path.isfile(tmp_path / "models" / "optimizer_3.pth")
@@ -60,10 +60,12 @@ def test_checkpoint_files_round_trip_with_the_reference_manager(tmp_path):
     for net, sd in mine.get_model_state().items():
         for k, v in sd.items():
             assert th.equal(other.get_model_state()[net][k], v)
-    if ref_import.reference_available():  # the reference's own manager loads the same file (trainer_base.py:703-705)
-        ns = ref_import.import_reference()
-        _, ref_mgr = ref_import.make_reference_manager(ns, 64, 96)
-        ref_mgr.set_model_state(th.load(X.models_file(tmp_path, 3)))
-        for net, sd in mine.get_model_state().items():
-            for k, v in sd.items():
-                assert th.equal(ref_mgr.get_model_state()[net][k], v), (net, k)
+    # the reference's own manager loads the same file (trainer_base.py:703-705): one state dict per net, each with exactly the
+    # names, shapes and dtypes of the reference manager's (its load_state_dict is strict)
+    ref = reference_managers()["dims_64_96"]["state"]
+    saved = th.load(X.models_file(tmp_path, 3))
+    assert sorted(saved) == sorted(ref)
+    for net, sd in saved.items():
+        assert layout(sd) == golden_layout(ref[net]), net
+        for k, v in sd.items():
+            assert th.equal(mine.get_model_state()[net][k], v), (net, k)

@@ -1,7 +1,7 @@
 """
 Edge cases of the path on the GPU (one segment per video, 27 segments = the ActivityNet maximum, single-frame / single-word
 sequences, a batch of one video, equal lengths): both product paths vs the CPU oracle, which tests/test_oracle_live_edges.py pins to
-the live reference on the same inputs.
+the reference's outputs on the same inputs.
 
 These cases were added AFTER the round's GPU budget was spent and have never run on a GPU.  Each runs in its own process
 (tests/edge_case_runner.py) so that a fault cannot poison the CUDA context of the other tests, and a failure is reported as XFAIL

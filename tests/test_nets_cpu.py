@@ -1,12 +1,15 @@
 """CPU-side checks of the host logic: parameter containers (reference state-dict names, flat storage), synthetic batches,
 cycle-loss weights."""
+import json
 import os
+from types import SimpleNamespace
 
 import pytest
 import torch as th
 
 from coot_videotext_b200 import synthetic as syn
 from coot_videotext_b200.nets import TransformerLegacyB200, entry_names
+from tests.util import GOLDEN_DIR
 
 
 def test_state_dict_names_match_reference_inventory():
@@ -22,56 +25,69 @@ def test_state_dict_names_match_reference_inventory():
         assert tuple(sd["embedding.pe"].shape) == (1000, 384)
 
 
-def _have_reference():
-    from oracle import ref_import
-    return ref_import.reference_available()  # /root/reference (build container) or the travelling copy oracle/_ref (GPU box)
+def reference_managers():
+    """What the reference's RetrievalModelManager reported for the shipped configs (tests/golden/make_golden_reference_meta.py)."""
+    return json.load(open(os.path.join(GOLDEN_DIR, "reference_managers.json")))
 
 
-@pytest.mark.skipif(not _have_reference(), reason="reference tree not available (python oracle/make_ref.py)")
+def golden_layout(entries):
+    """{name: (shape, dtype)} of one net's [name, shape, dtype] list in the golden file."""
+    return {k: (tuple(shape), dtype) for k, shape, dtype in entries}
+
+
+def layout(sd):
+    return {k: (tuple(v.shape), str(v.dtype)) for k, v in sd.items()}
+
+
+def _config(reads):
+    """The reference RetrievalConfig as far as it was read: attributes as a namespace, indexed entries as a dict."""
+    if not isinstance(reads, dict):
+        return reads
+    if "__items__" in reads:
+        return {k: _config(v) for k, v in reads["__items__"].items()}
+    return SimpleNamespace(**{k: _config(v) for k, v in reads.items()})
+
+
 @pytest.mark.parametrize("yaml_name", ["anet_coot.yaml", "yc2_100m_coot.yaml", "yc2_2d3d_coot.yaml"])
 def test_manager_constructed_from_the_shipped_configs_matches_the_reference_manager(yaml_name):
-    """RetrievalModelManager(cfg) with the reference's own RetrievalConfig objects of the three shipped experiments: same
-    state-dict names / shapes, same optimizer parameter groups (names, order, decay_mult / lr_mult), dropout taken from the config,
-    is_autocast_enabled() reporting like nntrainer/models/model_manager_base.py:31-38."""
-    from oracle import ref_import
+    """RetrievalModelManager(cfg) with the values of the reference's own RetrievalConfig objects of the three shipped experiments:
+    same state-dict names / shapes / dtypes as the reference manager, same optimizer parameter groups (names, order, decay_mult / lr_mult),
+    dropout taken from the config, is_autocast_enabled() reporting like nntrainer/models/model_manager_base.py:31-38."""
     from coot_videotext_b200.model_retrieval import RetrievalModelManager
-    ns = ref_import.import_reference()
-    d = ns.load_yaml_config_file(os.path.join(ref_import.REFERENCE_ROOT, "config/retrieval/paper2020", yaml_name))
-    d.update(use_cuda=False)
-    cfg = ns.RetrievalConfig(d)
-    ref = ns.RetrievalModelManager(cfg)
+    ref = reference_managers()[yaml_name]
+    cfg = _config(ref["config_reads"])
     mine = RetrievalModelManager(cfg)
-    rs, ms = ref.get_model_state(), mine.get_model_state()
-    assert list(rs) == list(ms)
-    for net in rs:
-        assert {k: tuple(v.shape) for k, v in rs[net].items()} == {k: tuple(v.shape) for k, v in ms[net].items()}, net
-    rp, rn, rf = ref.get_all_params()
+    ms = mine.get_model_state()
+    assert list(ms) == ref["nets"]
+    for net in ms:
+        assert layout(ms[net]) == golden_layout(ref["state"][net]), net
     mp, mn, mf = mine.get_all_params()
-    assert rn == mn and len(rp) == len(mp) == len(mf)
-    for a, b in zip(rp, mp):
-        assert a["decay_mult"] == b["decay_mult"] and a["lr_mult"] == b["lr_mult"] and a["params"].shape == b["params"].shape
-    for net in rs:
+    assert mn == [g[0] for g in ref["param_groups"]] and len(ref["param_groups"]) == len(mp) == len(mf)
+    for (_, decay_mult, lr_mult, shape), b in zip(ref["param_groups"], mp):
+        assert decay_mult == b["decay_mult"] and lr_mult == b["lr_mult"] and list(b["params"].shape) == shape
+    for net in ms:
         c = cfg.model_cfgs[net]
         assert mine.net_dropout[net][0] == c.selfatn.dropout
-    assert mine.is_autocast_enabled() == ref.is_autocast_enabled()
+    assert mine.is_autocast_enabled() == ref["autocast"]["train"]
     mine.set_all_models_eval()
-    ref.set_all_models_eval()
-    assert mine.is_autocast_enabled() == ref.is_autocast_enabled()
+    assert mine.is_autocast_enabled() == ref["autocast"]["eval"]
 
 
-@pytest.mark.skipif(not _have_reference(), reason="reference tree not available (python oracle/make_ref.py)")
 def test_state_dict_round_trips_with_the_reference_modules():
-    from oracle import ref_import
-    ns = ref_import.import_reference()
-    _, mgr = ref_import.make_reference_manager(ns, 64, 96)
+    """A checkpoint with the reference manager's state-dict layout loads into the drop-in, and the drop-in's state dict has exactly
+    that layout (names, shapes, dtypes), which is what the reference's strict load_state_dict requires."""
     from coot_videotext_b200.model_retrieval import RetrievalModelManager
+    ref = reference_managers()["dims_64_96"]["state"]
+    g = th.Generator().manual_seed(0)
+    state = {net: {k: th.randn(shape, generator=g).to(getattr(th, dtype.split(".")[-1])) for k, shape, dtype in entries}
+             for net, entries in ref.items()}
     mine = RetrievalModelManager(vid_feat_dim=64, text_feat_dim=96)
-    state = mgr.get_model_state()
     mine.set_model_state(state)  # reference checkpoint -> drop-in
     for net in state:
         for k, v in state[net].items():
             assert th.equal(mine.model_dict[net].state_dict()[k], v), (net, k)
-        mgr.model_dict[net].load_state_dict(mine.model_dict[net].state_dict())  # and back, strict
+    for net, sd in mine.get_model_state().items():  # and back
+        assert layout(sd) == golden_layout(ref[net]), net
 
 
 def test_flat_storage_survives_load_and_apply():

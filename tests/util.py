@@ -18,9 +18,9 @@ def hash_name(name: str) -> int:
     return h
 
 
-def grad_sample_index(name: str, numel: int) -> np.ndarray:
+def grad_sample_index(name: str, numel: int, samples: int = GRAD_SAMPLES) -> np.ndarray:
     rng = np.random.default_rng(abs(hash_name(name)) % (2 ** 32))
-    return rng.integers(0, numel, size=min(GRAD_SAMPLES, numel))
+    return rng.integers(0, numel, size=min(samples, numel))
 
 
 def rel_inf(a, b) -> float:
